@@ -229,6 +229,61 @@ def fft_backend(ol):
         return "in-repo fp32 radix-4 Stockham (FFTW unavailable)"
 
 
+def band_outputs(bands, counts, t_last_ms):
+    """What a caller of the timed path holds after its last step, per band: the counts of the last push's result, the complete
+    transmission mailbox, the live signal map, the spectrogram rows completed during that step, and the Averager output and noise
+    threshold the detector compared against. Integers and times as float64, dB values as float32."""
+    import numpy as np
+
+    out = []
+    for band, c in zip(bands, counts):
+        tx = band.get_transmissions()
+        keys, first, last, power = band.get_signals(cap=4096)
+        times = [np.zeros(0, np.int64)]
+        rows = [np.zeros((0, max(band.cfg.spectrogram_out_size, 1)), np.int8)]
+        while True:  # consume the band's row list; rows stamped before the last step belong to earlier steps
+            t, _, r = band.get_spectrogram(cap=256)
+            if len(t) == 0:
+                break
+            keep = t >= int(t_last_ms)
+            times.append(t[keep])
+            rows.append(r[keep])
+        _, avg, _, _ = band.get_averager()
+        thr, _, _ = band.get_noise()
+        out.append({
+            "result_counts": np.array(c, np.float64),  # n_transmissions, n_detect_entries, n_spectrogram_rows, n_transmissions_total
+            "transmissions": np.array(tx, np.float64).reshape(-1, 4),  # shift_hz, flush, key, power
+            "signals": np.stack([keys, first, last, power], axis=1).astype(np.float64),  # key, first_ms, last_ms, power
+            "spectrogram_times_ms": np.concatenate(times).astype(np.float64),
+            "spectrogram_rows": np.concatenate(rows).astype(np.float32),
+            "averager_db": avg,
+            "noise_threshold_db": thr,
+        })
+    return out
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(directory, per_band):
+    """DIR/band<b>_<name>.npy for every band; above DUMP_BUDGET_BYTES in all, a fixed seeded sample of whole bands is written."""
+    import numpy as np
+
+    sizes = [sum(a.nbytes for a in d.values()) for d in per_band]
+    keep = list(range(len(per_band)))
+    if sum(sizes) > DUMP_BUDGET_BYTES:
+        keep, total = [], 0
+        for b in np.random.default_rng(0).permutation(len(per_band)):
+            if total + sizes[b] <= DUMP_BUDGET_BYTES:
+                keep.append(int(b))
+                total += sizes[b]
+        keep.sort()
+    os.makedirs(directory, exist_ok=True)
+    for b in keep:
+        for name, a in per_band[b].items():
+            np.save(os.path.join(directory, f"band{b}_{name}.npy"), a)
+
+
 def run_reference(args, rank, world):
     """Reference arm: the CPU restatement of the reference path (oracle port, fp32), all host threads."""
     if rank != 0:
@@ -301,6 +356,8 @@ def main():
     ap.add_argument("--sweep", action="store_true", help="config 5: run T in {64, 256, 1024, 4096} and report all four")
     ap.add_argument("--skip-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--skip-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the bands returned for the last timed step of the device-resident run as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b2s" else max(args.warmup, 1)
 
@@ -352,8 +409,9 @@ def main():
             return int(HOP_CENTRES_MHZ[b % 8] * 1e6)
         return 150_000_000 + 1_000_000 * (rank * n_bands + b)
 
-    def run(T, steps, warmup, on_device, hop=False):
-        """One measurement: n_bands bands, `steps` timed steps of T frames per band. Returns (ms max over ranks, summed profile, clocks, stats)."""
+    def run(T, steps, warmup, on_device, hop=False, capture=False):
+        """One measurement: n_bands bands, `steps` timed steps of T frames per band. Returns (ms max over ranks, summed profile, clocks, stats);
+        with `capture`, stats["outputs"] holds what every band returned for the last timed step (see band_outputs)."""
         iq_dev = [synth.make_iq_int8_torch(n, T, tones_for(T), seed=synth.seed_for(args.config, rank * n_bands + b), quiet_frames=LEARN, device=dev) for b in range(n_bands)]
         hosts = None
         if not on_device:
@@ -402,14 +460,18 @@ def main():
         for _ in range(steps):
             step()
         n_tx, n_ent = 0, 0
+        counts = []
         for band in bands:  # async result mode: every push's kernels AND bookkeeping are complete before the clock stops
             band.sync(res)
             n_tx += res.n_transmissions_total
             n_ent += res.n_detect_entries
+            counts.append((res.n_transmissions, res.n_detect_entries, res.n_spectrogram_rows, res.n_transmissions_total))
         e1.record(main_stream)
         barrier()
         clocks = sampler.stop()
         ms = e0.elapsed_time(e1)
+        # before the untimed profiling pushes below change the bands' state
+        outputs = band_outputs(bands, counts, t_ms - T * period) if capture else None
         profs = [band.get_profile(reset=True) for band in bands]
         cta = None
         if on_device and n_bands == 1:
@@ -426,7 +488,7 @@ def main():
         del iq_dev, hosts
         agg = {k: sum(getattr(p, k) for p in profs) for k in ("spectral_ms", "detect_ms", "window_ms", "tracker_host_ms", "track_ms", "spectral_launches", "detect_launches",
                                                               "window_launches", "track_launches", "track_evals", "track_events", "track_best_index", "pushes", "h2d_bytes", "d2h_bytes")}
-        return reduce_step_time(ms, dev), agg, clocks, {"n_tx": n_tx, "n_entries": n_ent, "cta": cta}
+        return reduce_step_time(ms, dev), agg, clocks, {"n_tx": n_tx, "n_entries": n_ent, "cta": cta, "outputs": outputs}
 
     peak, peak_src = measured_peaks()
 
@@ -446,7 +508,9 @@ def main():
 
     T = wl["frames"]
     # ---- device-resident run (value + roofline) ----
-    ms, agg, clocks, stats = run(T, args.steps, args.warmup, True, hop=args.hop)
+    ms, agg, clocks, stats = run(T, args.steps, args.warmup, True, hop=args.hop, capture=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, stats["outputs"])
     head = summarise(T, args.steps, ms, agg, hop=args.hop)
     samples_step = n_bands * T * n
     k1_ms, k2_ms = head["k1_ms"], head["k2_ms"]

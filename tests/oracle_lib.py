@@ -3,6 +3,7 @@ TEST INFRASTRUCTURE ONLY — nothing under rtl-sdr-scanner-cpp_b200/ imports thi
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -13,6 +14,7 @@ from conftest import ROOT, load_b2s
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 ORACLE_SO = os.path.join(ORACLE_DIR, "liboracle.so")
 REF_SO = os.path.join(ORACLE_DIR, "_ref", "libref.so")
+REF_OUTPUTS = os.path.join(ROOT, "tests", "golden", "reference_outputs.npz")
 MAX_TX = 64
 
 b2s = load_b2s()
@@ -122,6 +124,46 @@ def ref():
 
 def _p(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+# ---------------- what the reference's compiled objects returned, stored under tests/golden ----------------
+# The tests that compare with the reference read its outputs from REF_OUTPUTS, so they run where the reference is absent.
+# tests/golden/make_reference_outputs.py regenerates the file by calling every record_<name>() of those test modules with
+# oracle/_ref/libref.so; record_<name>() builds exactly the inputs its test builds. Arrays too large to store are stored as
+# one digest per row: the comparisons they stand for are bit for bit.
+_recorded = None
+
+
+def digest(a) -> int:
+    """64-bit digest of an array's bytes (or of a bytes object)."""
+    b = a if isinstance(a, bytes) else np.ascontiguousarray(a).tobytes()
+    return int.from_bytes(hashlib.blake2b(b, digest_size=8).digest(), "little")
+
+
+def digests(rows) -> np.ndarray:
+    return np.array([digest(r) for r in rows], dtype=np.uint64)
+
+
+def recorded(name: str) -> dict:
+    """The arrays record_<name>() stored, keyed by field."""
+    global _recorded
+    if _recorded is None:
+        with np.load(REF_OUTPUTS, allow_pickle=False) as z:
+            _recorded = {k: z[k] for k in z.files}
+    out = {k.split(".", 1)[1]: v for k, v in _recorded.items() if k.split(".", 1)[0] == name}
+    assert out, f"{name} is not in {os.path.relpath(REF_OUTPUTS, ROOT)}: regenerate it with tests/golden/make_reference_outputs.py"
+    return out
+
+
+def pack_lists(lists) -> dict:
+    """Per-frame [(shift_hz, flush)] lists -> count per frame + all pairs (int32)."""
+    pairs = [p for lst in lists for p in lst]
+    return {"count": np.array([len(lst) for lst in lists], np.int32), "pairs": np.array(pairs, np.int32).reshape(-1, 2)}
+
+
+def unpack_lists(rec: dict):
+    ends = np.cumsum(rec["count"])
+    return [[(int(f), int(fl)) for f, fl in rec["pairs"][e - c : e]] for c, e in zip(rec["count"], ends)]
 
 
 def have_ref_blocks() -> bool:

@@ -1,7 +1,7 @@
 """Pins the CPU oracle (oracle/scan_oracle.cpp):
   (1) against the reference's own gtest known-answer vectors (tests/golden/reference_kats.json), and
-  (2) against the reference's own objects compiled from /root/reference (oracle/_ref/libref.so), bit for bit,
-      on random inputs — for every hot-path piece that the reference can be built for here (SURVEY.md §8c).
+  (2) against what the reference's own compiled objects returned for random inputs (stored in tests/golden/reference_outputs.npz),
+      bit for bit — for every hot-path piece that the reference can be built for (SURVEY.md §8c).
 CPU only (-m "not gpu")."""
 import ctypes as C
 import json
@@ -14,7 +14,7 @@ import oracle_lib as ol
 from conftest import ROOT
 
 G = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_kats.json")))
-needs_ref = pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref/libref.so not built (needs /root/reference)")
+needs_ref = pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref/libref.so not built (needs the reference sources)")
 KINDS = ["orc"] + (["ref"] if ol.have_ref() else [])
 
 
@@ -115,63 +115,115 @@ def test_averager_fixture_kat(kind):
 
 
 # ---------------- oracle == compiled reference, bit for bit, on random data ----------------
-@needs_ref
-@pytest.mark.parametrize("size,group", [(5, 3), (64, 21), (1000, 21), (4096, 21), (33, 1)])
-def test_averager_matches_reference_bitwise(size, group):
+# The reference's outputs are read from tests/golden/reference_outputs.npz (oracle_lib.recorded); record_<name>() made them from
+# the compiled reference on the same inputs.
+AVERAGER_SHAPES = [(5, 3), (64, 21), (1000, 21), (4096, 21), (33, 1)]
+AVERAGE_SHAPES = [(9, 5), (100, 21), (4096, 21), (16384, 21), (50, 1), (10, 21), (7, 4)]
+
+
+def _averager_steps(av, size, group):
+    """Pushes the random rows of the test; yields (average, data) after every push."""
     rng = np.random.default_rng(size * 131 + group)
-    a, b = ol.CpuAverager(size, group, "orc"), ol.CpuAverager(size, group, "ref")
     for step in range(3 * group + 7):
         if step == 2 * group + 1:
-            a.reset(), b.reset()
-        row = (rng.standard_normal(size) * 30 - 20).astype(np.float32)
-        a.push(row), b.push(row)
-        assert a.average().tobytes() == b.average().tobytes()
-        assert a.data().tobytes() == b.data().tobytes()
+            av.reset()
+        av.push((rng.standard_normal(size) * 30 - 20).astype(np.float32))
+        yield av.average(), av.data()
 
 
-@needs_ref
-@pytest.mark.parametrize("size,group", [(9, 5), (100, 21), (4096, 21), (16384, 21), (50, 1), (10, 21), (7, 4)])
-def test_average_matches_reference_bitwise(size, group):
+def record_averager_bitwise():
+    out = {}
+    for size, group in AVERAGER_SHAPES:
+        steps = list(_averager_steps(ol.CpuAverager(size, group, "ref"), size, group))
+        out[f"avg_{size}_{group}"] = ol.digests(a for a, _ in steps)
+        out[f"data_{size}_{group}"] = ol.digests(d for _, d in steps)
+    return out
+
+
+@pytest.mark.parametrize("size,group", AVERAGER_SHAPES)
+def test_averager_matches_reference_bitwise(size, group):
+    want = ol.recorded("averager_bitwise")
+    assert len(want[f"avg_{size}_{group}"]) == 3 * group + 7
+    for step, (avg, data) in enumerate(_averager_steps(ol.CpuAverager(size, group, "orc"), size, group)):
+        assert ol.digest(avg) == want[f"avg_{size}_{group}"][step], step
+        assert ol.digest(data) == want[f"data_{size}_{group}"][step], step
+
+
+def _average_inputs(size, group):
     rng = np.random.default_rng(size + group)
     for scale in (1.0, 40.0):
-        x = (rng.standard_normal(size) * scale - 7).astype(np.float32)
-        assert ol.cpu_average(x, group, "orc").tobytes() == ol.cpu_average(x, group, "ref").tobytes()
-    x = np.full(size, -100, np.float32)
-    assert ol.cpu_average(x, group, "orc").tobytes() == ol.cpu_average(x, group, "ref").tobytes()
+        yield (rng.standard_normal(size) * scale - 7).astype(np.float32)
+    yield np.full(size, -100, np.float32)
 
 
-@needs_ref
-def test_collection_utils_match_reference_random():
+def record_average_bitwise():
+    return {f"{size}_{group}": ol.digests(ol.cpu_average(x, group, "ref") for x in _average_inputs(size, group)) for size, group in AVERAGE_SHAPES}
+
+
+@pytest.mark.parametrize("size,group", AVERAGE_SHAPES)
+def test_average_matches_reference_bitwise(size, group):
+    want = ol.recorded("average_bitwise")[f"{size}_{group}"]
+    got = ol.digests(ol.cpu_average(x, group, "orc") for x in _average_inputs(size, group))
+    assert np.array_equal(got, want)
+
+
+def _collection_cases():
     rng = np.random.default_rng(7)
-    O, R = ol.oracle(), ol.ref()
     for _ in range(300):
         n = int(rng.integers(1, 200))
         d = rng.integers(-5, 6, n).astype(np.float32)  # many ties: first-maximum rule matters
         idx, grp = int(rng.integers(0, n)), int(rng.integers(0, 64))
-        p = d.ctypes.data_as(C.c_void_p)
-        assert O.orc_get_max_index(p, n, idx, grp) == R.ref_get_max_index(p, n, idx, grp)
         v = rng.integers(0, 8, int(rng.integers(1, 30))).astype(np.int32)
-        pv = v.ctypes.data_as(C.c_void_p)
-        assert O.orc_most_frequent_value(pv, len(v)) == R.ref_most_frequent_value(pv, len(v))
         keys = np.unique(rng.integers(0, 500, int(rng.integers(0, 12)))).astype(np.int32)
-        pk = keys.ctypes.data_as(C.c_void_p)
-        fo, fr = C.c_int(-1), C.c_int(-1)
         index, margin = int(rng.integers(-10, 510)), int(rng.integers(0, 140))
-        ro = O.orc_contains_with_margin(pk, len(keys), index, margin, C.byref(fo))
-        rr = R.ref_contains_with_margin(pk, len(keys), index, margin, C.byref(fr))
-        assert ro == rr and (not ro or fo.value == fr.value)
+        yield d, idx, grp, v, keys, index, margin
 
 
-@needs_ref
-def test_radio_utils_match_reference_random():
+def _collection_results(kind):
+    """[max index, most frequent value, contains, found key (-1 when not contained)] per case."""
+    L = _lib(kind)
+    out = []
+    for d, idx, grp, v, keys, index, margin in _collection_cases():
+        found = C.c_int(-1)
+        contains = getattr(L, f"{kind}_contains_with_margin")(keys.ctypes.data_as(C.c_void_p), len(keys), index, margin, C.byref(found))
+        out.append((getattr(L, f"{kind}_get_max_index")(d.ctypes.data_as(C.c_void_p), len(d), idx, grp),
+                    getattr(L, f"{kind}_most_frequent_value")(v.ctypes.data_as(C.c_void_p), len(v)), contains, found.value if contains else -1))
+    return np.array(out, np.int64)
+
+
+def record_collection_utils():
+    return {"results": _collection_results("ref")}
+
+
+def test_collection_utils_match_reference_random():
+    got, want = _collection_results("orc"), ol.recorded("collection_utils")["results"]
+    assert got.shape == want.shape
+    for i in range(len(want)):
+        assert tuple(got[i]) == tuple(want[i]), i
+
+
+def _tuned_cases():
     rng = np.random.default_rng(11)
-    O, R = ol.oracle(), ol.ref()
-    for _ in range(2000):
-        f, step = int(rng.integers(-2_000_000, 2_000_000)), int(rng.integers(1, 100_000))
-        assert O.orc_get_tuned_frequency(f, step) == R.ref_get_tuned_frequency(f, step)
-    for fs in (250_000, 1_024_000, 2_048_000, 2_400_000, 10_000_000, 20_000_000, 40_000_000, 61_440_000):
-        for step in (100, 250, 625, 1000):
-            assert O.orc_get_fft(fs, step) == R.ref_get_fft(fs, step)
+    return [(int(rng.integers(-2_000_000, 2_000_000)), int(rng.integers(1, 100_000))) for _ in range(2000)]
+
+
+FFT_CASES = [(fs, step) for fs in (250_000, 1_024_000, 2_048_000, 2_400_000, 10_000_000, 20_000_000, 40_000_000, 61_440_000) for step in (100, 250, 625, 1000)]
+
+
+def _radio_results(kind):
+    L = _lib(kind)
+    return {"tuned": np.array([getattr(L, f"{kind}_get_tuned_frequency")(f, step) for f, step in _tuned_cases()], np.int64),
+            "fft": np.array([getattr(L, f"{kind}_get_fft")(fs, step) for fs, step in FFT_CASES], np.int64)}
+
+
+def record_radio_utils():
+    return _radio_results("ref")
+
+
+def test_radio_utils_match_reference_random():
+    got, want = _radio_results("orc"), ol.recorded("radio_utils")
+    assert np.array_equal(got["tuned"], want["tuned"])
+    assert np.array_equal(got["fft"], want["fft"])
 
 
 @needs_ref

@@ -1,6 +1,7 @@
 """Randomised PSD scenes through the REFERENCE'S OWN compiled NoiseLearner -> Transmission objects and through the oracle
 (same rows, same injected clock): NoiseLearner rows bit for bit, the FrequencyFlush list of every frame identical. Many
-concurrent carriers, drifting and overlapping, near the band edges, ignored ranges, scan-range limits, odd / even group sizes."""
+concurrent carriers, drifting and overlapping, near the band edges, ignored ranges, scan-range limits, odd / even group sizes.
+What the reference objects returned is read from tests/golden/reference_outputs.npz (record_random_scenes made it)."""
 import numpy as np
 import pytest
 
@@ -8,8 +9,6 @@ import oracle_lib as ol
 from conftest import load_b2s
 
 b2s = load_b2s()
-
-pytestmark = pytest.mark.skipif(not (ol.have_ref() and ol.have_ref_blocks()), reason="oracle/_ref/libref.so (reference blocks) not built: needs /root/reference")
 
 PERIOD_MS = 100.0  # NOISE_LEARNING_TIME = 2000 ms (config.h:24) = 21 frames of this clock
 T0 = 1_700_000_000_000
@@ -46,14 +45,32 @@ def _scene(seed):
     return cfg, psd, frames, bw
 
 
-@pytest.mark.parametrize("seed", range(16))
+SEEDS = range(16)
+
+
+def record_random_scenes():
+    out = {}
+    for seed in SEEDS:
+        cfg, psd, frames, bw = _scene(seed)
+        ref = ol.RefBlocksChain(cfg, T0, bw, with_spectrogram=False)
+        rows, lists = [], []
+        for k in range(frames):
+            q, tx = ref.push_row(psd[k], T0 + int(np.floor(k * PERIOD_MS + 0.5)))
+            rows.append(q)
+            lists.append(tx)
+        out |= {f"{seed}_rows": ol.digests(rows)} | {f"{seed}_{k}": v for k, v in ol.pack_lists(lists).items()}
+    return out
+
+
+@pytest.mark.parametrize("seed", SEEDS)
 def test_random_scene_against_the_reference_objects(seed):
     cfg, psd, frames, bw = _scene(seed)
     r = ol.OracleChain(cfg).push(psd, frames, T0, PERIOD_MS, dense=("noise_sub_db",), psd_rows=True)
-    ref = ol.RefBlocksChain(cfg, T0, bw, with_spectrogram=False)
-    for k in range(frames):
-        q, tx = ref.push_row(psd[k], T0 + int(np.floor(k * PERIOD_MS + 0.5)))
-        assert np.array_equal(q.view(np.uint32), r.noise_sub_db[k].view(np.uint32)), f"seed {seed}: NoiseLearner row {k}"
+    want = ol.recorded("random_scenes")
+    lists = ol.unpack_lists({"count": want[f"{seed}_count"], "pairs": want[f"{seed}_pairs"]})
+    assert len(lists) == frames
+    for k, tx in enumerate(lists):
+        assert ol.digest(r.noise_sub_db[k]) == want[f"{seed}_rows"][k], f"seed {seed}: NoiseLearner row {k}"
         assert _same_up_to_ties(tx, r.frame_tx[k]), f"seed {seed}: list of frame {k}: reference {tx} oracle {r.frame_tx[k]}"
 
 

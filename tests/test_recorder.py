@@ -25,14 +25,23 @@ def test_resampler_factors_match_the_reference_vectors():
         if max(max(p) for p in want) < 100000:
             assert b2s.get_resamplers_factors(fs, bw, thr) == want, (fs, bw)
     assert b2s.get_resamplers_factors(40_000_000, 32_000) == [(1, 25), (1, 50)]  # BASELINE config 4 (SURVEY.md 8d)
-    if ol.have_ref():
-        import ctypes as C
+    for (fs, bw), want in zip(RESAMPLER_CASES, ol.unpack_lists(ol.recorded("resamplers_factors")), strict=True):
+        assert ro.resamplers_factors(fs, bw) == want == b2s.get_resamplers_factors(fs, bw)
 
-        buf = np.zeros(32, np.int32)
-        for fs, bw in ((40_000_000, 32_000), (20_000_000, 32_000), (2_048_000, 32_000), (1_024_000, 20_000), (2_400_000, 12_500)):
-            k = ol.ref().ref_get_resamplers_factors(fs, bw, 125, buf.ctypes.data_as(C.c_void_p), 16)
-            want = [(int(buf[2 * i]), int(buf[2 * i + 1])) for i in range(k)]
-            assert ro.resamplers_factors(fs, bw) == want == b2s.get_resamplers_factors(fs, bw)
+
+RESAMPLER_CASES = ((40_000_000, 32_000), (20_000_000, 32_000), (2_048_000, 32_000), (1_024_000, 20_000), (2_400_000, 12_500))
+
+
+def record_resamplers_factors():
+    """getResamplersFactors of the compiled reference (threshold 125)."""
+    import ctypes as C
+
+    buf = np.zeros(32, np.int32)
+    lists = []
+    for fs, bw in RESAMPLER_CASES:
+        k = ol.ref().ref_get_resamplers_factors(fs, bw, 125, buf.ctypes.data_as(C.c_void_p), 16)
+        lists.append([(int(buf[2 * i]), int(buf[2 * i + 1])) for i in range(k)])
+    return ol.pack_lists(lists)
 
 
 def test_tap_design_known_properties():

@@ -1,6 +1,6 @@
 """Scanner hop policy and recorder assignment (SURVEY.md §8(f)#3), CPU only. The product's host state machine (csrc/scan_policy.h, through
 the C ABI) against (1) the reference's gtest vectors for getRangeSplitSampleRate / splitRange (tests/test_radio_utils.cpp:105-132),
-(2) the compiled reference functions where /root/reference is present, and (3) an independent Python restatement of
+(2) what the compiled reference functions returned (tests/golden/reference_outputs.npz), and (3) an independent Python restatement of
 Scanner::worker (scanner.cpp:36-64) and SdrDevice::updateRecordings (sdr_device.cpp:82-144) on randomised notification sequences."""
 import ctypes as C
 
@@ -20,14 +20,26 @@ def test_range_split_against_reference_vectors():
         # splitRange with the split rate given directly: a policy whose device sample rate maps onto itself
         assert b2s.get_range_split_sample_rate(fs) == fs
         assert b2s.ScanPolicy([(lo, hi)], fs, 1).ranges() == [tuple(r) for r in want]
-    if ol.have_ref():
-        R = ol.ref()
-        buf = np.zeros(512, np.int32)
-        for fs in (2_048_000, 20_480_000, 250_000, 1_920_000):
-            split = R.ref_get_range_split_sample_rate(fs)
-            assert b2s.get_range_split_sample_rate(fs) == split
-            k = R.ref_split_range(144_000_000, 174_000_000, split, buf.ctypes.data_as(C.c_void_p), 256)
-            assert b2s.ScanPolicy([(144_000_000, 174_000_000)], fs, 2).ranges() == [(int(buf[2 * i]), int(buf[2 * i + 1])) for i in range(k)]
+    want = ol.recorded("range_split")
+    for fs, split, ranges in zip(SPLIT_RATES, want["rate"], ol.unpack_lists(want), strict=True):
+        assert b2s.get_range_split_sample_rate(fs) == split
+        assert b2s.ScanPolicy([(144_000_000, 174_000_000)], fs, 2).ranges() == ranges
+
+
+SPLIT_RATES = (2_048_000, 20_480_000, 250_000, 1_920_000)
+
+
+def record_range_split():
+    """getRangeSplitSampleRate and splitRange(144-174 MHz) of the compiled reference."""
+    R = ol.ref()
+    buf = np.zeros(512, np.int32)
+    rates, lists = [], []
+    for fs in SPLIT_RATES:
+        split = R.ref_get_range_split_sample_rate(fs)
+        k = R.ref_split_range(144_000_000, 174_000_000, split, buf.ctypes.data_as(C.c_void_p), 256)
+        rates.append(split)
+        lists.append([(int(buf[2 * i]), int(buf[2 * i + 1])) for i in range(k)])
+    return {"rate": np.array(rates, np.int64), **ol.pack_lists(lists)}
 
 
 class PyScanner:
